@@ -9,6 +9,7 @@ cell steps, all 12 hidden states emitted (SURVEY.md section 8d).
 
   python bench.py [--gpus N --steps K --warmup W]      our arm (N>1 under torchrun, one rank per GPU)
   python bench.py --impl reference ...                 the reference's CPU path (oracle port) on the host cores
+  python bench.py ... --dump-outputs DIR               also write what the last timed step returned (see `dump_outputs`)
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for every field.
 """
@@ -33,6 +34,24 @@ N_NODES, N_EDGES, F_IN, HORIZON, HIDDEN, K_HOPS = 207, 1722, 2, 12, 32, 2
 BYTES_PER_SNAPSHOT = HORIZON * N_NODES * F_IN * 4 + HORIZON * N_NODES * HIDDEN * 4  # 337 824 B
 # algorithmic FLOPs per snapshot (z/r share the diffusion): 9 GEMMs 207x34x32 + 2 dirs x (34+32) diffusion + gates
 FLOPS_PER_SNAPSHOT = HORIZON * (9 * 2 * N_NODES * 34 * HIDDEN + 2 * 2 * N_EDGES * (34 + 32) + 10 * N_NODES * HIDDEN)
+DUMP_WINDOWS = 128    # windows of the last step --dump-outputs writes: 128 x 318 KB of hidden states = 41 MB
+
+
+def dump_rows(windows):
+    """The fixed, seeded sample of a step's windows that --dump-outputs writes (all of them if there are at most DUMP_WINDOWS)."""
+    return torch.randperm(windows, generator=torch.Generator().manual_seed(0))[:DUMP_WINDOWS].sort().values
+
+
+def dump_outputs(out_dir, hidden, prediction):
+    """hidden_states.npy: float32 (DUMP_WINDOWS, 12, 207, 32), BatchedDCRNN.forward's output for the sampled windows of the last
+    timed device-resident step; prediction.npy: float32 (DUMP_WINDOWS, 207), the Linear head's output for the same windows in
+    the last timed end-to-end step (absent if that leg failed).  The inputs depend only on the arguments, so two builds run
+    with the same arguments can be compared file by file."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "hidden_states.npy"), hidden.numpy())
+    if prediction is not None:
+        np.save(os.path.join(out_dir, "prediction.npy"), prediction.numpy())
 
 
 def peaks():
@@ -360,6 +379,10 @@ def run_ours(args):
     launches = _lib.launch_count() - l0
     ms_total = e0.elapsed_time(e1)
     clocks = sampler.stop() if rank == 0 else None
+    dump = args.dump_outputs is not None and rank == 0
+    if dump:
+        rows = dump_rows(B)
+        hidden = out[rows.to(dev)].cpu()
     t = torch.tensor([ms_total], device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -427,6 +450,9 @@ def run_ours(args):
         if world > 1:
             raise                                   # ranks must stay in lock step around collectives: fail loudly under torchrun
         e2e["error"] = f"{type(e).__name__}: {e}"
+    if dump:
+        # step i of run_e2e leaves its prediction in pred_host[i % 2]
+        dump_outputs(args.dump_outputs, hidden, pred_host[(args.steps - 1) % 2][rows] if e2e["value"] is not None else None)
 
     # ---- roofline of the dominant kernel (k_dcrnn_seq_tc = the whole step) ---------------------------------------
     achieved_gbs = B * BYTES_PER_SNAPSHOT / (ms_step * 1e-3) / 1e9
@@ -651,7 +677,13 @@ def main():
     ap.add_argument("--no-train", action="store_true")
     ap.add_argument("--no-refgpu", action="store_true")
     ap.add_argument("--no-hostwin", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last step's outputs for a fixed "
+                    "sample of its windows as DIR/hidden_states.npy and DIR/prediction.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of our arm (--impl ours)")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

@@ -61,9 +61,14 @@ def main():
     torch.manual_seed(1)
     m1 = dc.DCRNN(2, 32, 2)
     x1, h1 = torch.randn(207, 2), torch.randn(207, 32) * 0.5
+    # one thread: the dense-adjacency in-degrees are a (1 x 207) @ (207 x 207) product whose reduction MKL splits by thread
+    # count, so only a fixed count reproduces these bits on another machine (tests/test_goldens_cpu.py runs it the same way)
+    threads = torch.get_num_threads()
+    torch.set_num_threads(1)
     with torch.no_grad():
         o1 = m1(x1, ei_t, ew_t, h1)
         o1_now = m1(x1, ei_t)  # edge_weight None, H None
+    torch.set_num_threads(threads)
     save("dcrnn_cfg2_cell", edge_index=ei_t, edge_weight=ew_t, X=x1, H=h1, state=sd(m1), out=o1, out_noew_noh=o1_now, K=2)
     # K=1,3,4 on a small asymmetric graph (exercises the positional norm_in pairing and the Tx_0 quirk)
     ei_s, ew_s = small_graph(40, 150, 3)

@@ -4,7 +4,7 @@ replicas stay bit-identical after an optimizer step."""
 import os
 import socket
 
-import pytest
+import numpy as np
 import torch
 import torch.distributed as dist
 import torch.multiprocessing as mp
@@ -44,17 +44,26 @@ def _worker(rank, world, port, q):
     dist.destroy_process_group()
 
 
-def test_two_rank_gloo_flat_allreduce_and_sharding():
+def test_two_rank_gloo_flat_allreduce_and_sharding(monkeypatch):
+    # the CPU path on any machine: with a GPU visible, init_process_group would put rank r on cuda:r, and a one-GPU
+    # machine has no cuda:1 (the spawned workers read this environment; CUDA in this process is unaffected)
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")
     world, port = 2, _free_port()
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     procs = [ctx.Process(target=_worker, args=(r, world, port, q)) for r in range(world)]
     for p in procs:
         p.start()
-    res = sorted([q.get(timeout=120) for _ in range(world)], key=lambda t: t[0])
-    for p in procs:
-        p.join(timeout=60)
-        assert p.exitcode == 0
+    try:
+        res = sorted([q.get(timeout=120) for _ in range(world)], key=lambda t: t[0])
+        for p in procs:
+            p.join(timeout=60)
+            assert p.exitcode == 0
+    finally:
+        for p in procs:                     # a rank left waiting for a failed peer must not outlive the test
+            if p.is_alive():
+                p.kill()
+                p.join()
     (_, idx0, g0, avg0, w0, v0), (_, idx1, g1, avg1, w1, v1) = res
     assert sorted(idx0 + idx1) == list(range(20))                     # the shards partition the windows
     g0, g1, avg0, avg1 = (torch.tensor(t) for t in (g0, g1, avg0, avg1))
@@ -80,22 +89,21 @@ def test_masked_mae():
     assert abs(float(D.masked_mae_loss(y, t)) - 0.75) < 1e-6
 
 
-def test_masked_mae_matches_reference_example_util():
+def _mae_inputs(zero_frac):
+    """(prediction, target) of one masked-MAE case; a `zero_frac` share of the targets is 0 (missing)."""
+    rs = np.random.RandomState(int(zero_frac * 10))
+    y = rs.standard_normal((64, 207)).astype(np.float32)
+    y[rs.random_sample((64, 207)) < zero_frac] = 0.0
+    return torch.from_numpy(rs.standard_normal((64, 207)).astype(np.float32)), torch.from_numpy(y)
+
+
+def test_masked_mae_matches_reference_example_util(golden_dir):
     """The op-for-op form (the checker of the fused CUDA loss) against the unmodified reference function
-    examples/indexBatching/DCRNN/utils.py:10-18, loaded by path where /root/reference exists."""
-    import importlib.util
-    import os
-    path = "/root/reference/examples/indexBatching/DCRNN/utils.py"
-    if not os.path.isfile(path):
-        pytest.skip("/root/reference not present")
-    spec = importlib.util.spec_from_file_location("ref_dcrnn_utils", path)
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
-    torch.manual_seed(0)
+    examples/indexBatching/DCRNN/utils.py:10-18, whose results are stored in tests/golden/reference_data.pt
+    (tests/golden/make_goldens_parity.py)."""
+    ref = torch.load(os.path.join(golden_dir, "reference_data.pt"), weights_only=False)["masked_mae"]
     for zero_frac in (0.0, 0.3, 1.0):
-        y = torch.randn(64, 207)
-        y[torch.rand(64, 207) < zero_frac] = 0.0
-        p = torch.randn(64, 207)
-        a, b = D.masked_mae_loss_reference(p, y), ref.masked_mae_loss(p, y)
-        assert torch.equal(a, b)
+        p, y = _mae_inputs(zero_frac)
+        b = ref[zero_frac]
+        assert torch.equal(D.masked_mae_loss_reference(p, y), b)
         assert torch.equal(D.masked_mae_loss(p, y), b)          # CPU tensors take the op-for-op form

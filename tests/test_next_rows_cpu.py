@@ -1,13 +1,14 @@
 """Host-side tests of the SURVEY 8f rank 2/3 rows: StaticGraphTemporalSignalBatch (mirrors test/batch_test.py:120-134,
-:181-190) and the offline METR-LA / PEMS-BAY loaders (mirrors test/index_test.py:18-66 on synthetic archives; where
-/root/reference is present the unmodified reference loaders are run on the same files and must agree bit for bit)."""
+:181-190) and the offline METR-LA / PEMS-BAY loaders (mirrors test/index_test.py:18-66 on synthetic archives; what the
+unmodified reference loaders and iterators return on the same inputs is stored in tests/golden/reference_data.pt by
+tests/golden/make_goldens_parity.py and must be matched bit for bit)."""
+import hashlib
 import os
 
 import numpy as np
 import pytest
 import torch
 
-from oracle import refload
 from pytorch_geometric_temporal_b200.dataset import METRLADatasetLoader, PemsBayDatasetLoader, dense_to_sparse
 from pytorch_geometric_temporal_b200.signal import StaticGraphTemporalSignalBatch, temporal_signal_split
 
@@ -98,35 +99,33 @@ def test_offline_loader_errors(tmp_path):
         METRLADatasetLoader(raw_data_dir=str(tmp_path)).get_index_dataset()
 
 
-@pytest.mark.skipif(not refload.available(), reason="/root/reference not present")
+def _digest(t):
+    """SHA-256 of a tensor's dtype, shape and bytes: equal digests <=> bit-identical tensors of one dtype and shape."""
+    t = t.contiguous()
+    return hashlib.sha256(f"{t.dtype}{tuple(t.shape)}".encode() + t.numpy().tobytes()).hexdigest()
+
+
+@pytest.fixture(scope="module")
+def ref(golden_dir):
+    return torch.load(os.path.join(golden_dir, "reference_data.pt"), weights_only=False)
+
+
 @pytest.mark.parametrize("mod,name,prefix", [("dataset.metr_la", "METRLADatasetLoader", ""), ("dataset.pems_bay", "PemsBayDatasetLoader", "pems_")])
-def test_offline_loaders_match_reference(tmp_path, mod, name, prefix):
+def test_offline_loaders_match_reference(tmp_path, mod, name, prefix, ref):
+    """Our loaders against the outputs of the unmodified reference loaders on the same archive, stored as `_digest`s."""
     tmp = str(tmp_path)
-    _archive(tmp, 9, 2, 60, prefix)
-    open(os.path.join(tmp, "METR-LA.zip" if prefix == "" else "PEMS-BAY.zip"), "wb").close()      # the reference checks the zip exists
-    # the reference loader does `from ..signal import StaticGraphTemporalSignal`; its signal/__init__ pulls every iterator
-    # (PyG Batch/HeteroData), so expose just that one unmodified class on the path-only parent package refload registers
-    import sys
-    sig = refload.load("signal.static_graph_temporal_signal")
-    sys.modules["torch_geometric_temporal.signal"].StaticGraphTemporalSignal = sig.StaticGraphTemporalSignal
-    ref_cls = getattr(refload.load(mod), name)
+    _archive(tmp, 9, 2, 30, prefix)
+    want = ref["loaders"][prefix]
     ours_cls = METRLADatasetLoader if prefix == "" else PemsBayDatasetLoader
-    want, got = ref_cls(raw_data_dir=tmp).get_dataset(6, 6), ours_cls(raw_data_dir=tmp).get_dataset(6, 6)
-    assert want.snapshot_count == got.snapshot_count
-    for a, b in zip(want, got):
-        assert torch.equal(a.x, b.x) and torch.equal(a.y, b.y) and torch.equal(a.edge_index, b.edge_index) and torch.equal(a.edge_attr, b.edge_attr)
-    w = ref_cls(raw_data_dir=tmp, index=True).get_index_dataset(lags=6, batch_size=4)
+    got = [[_digest(getattr(b, k)) for k in ("x", "y", "edge_index", "edge_attr")] for b in ours_cls(raw_data_dir=tmp).get_dataset(6, 6)]
+    assert got == want["snapshots"]
     g = ours_cls(raw_data_dir=tmp, index=True).get_index_dataset(lags=6, batch_size=4)
     for i in range(3):
-        for (xa, ya), (xb, yb) in zip(w[i], g[i]):
-            assert torch.equal(xa, xb) and torch.equal(ya, yb)
-    for i in range(3, 7):
-        assert torch.equal(w[i], g[i])
+        assert [[_digest(x), _digest(y)] for x, y in g[i]] == want["index_batches"][i]
+    assert [_digest(t) for t in g[3:7]] == want["index_tensors"]
     # DistributedSampler shards
-    w = ref_cls(raw_data_dir=tmp, index=True).get_index_dataset(lags=6, batch_size=4, shuffle=True, world_size=2, ddp_rank=1)
     g = ours_cls(raw_data_dir=tmp, index=True).get_index_dataset(lags=6, batch_size=4, shuffle=True, world_size=2, ddp_rank=1)
-    for (xa, ya), (xb, yb) in zip(w[0], g[0]):
-        assert torch.equal(xa, xb) and torch.equal(ya, yb)
+    assert [[_digest(x), _digest(y)] for x, y in g[0]] == want["shard_batches"]
 
 
 # ---- SURVEY 8f rank 4: dynamic-graph iterators ------------------------------------------------------------------------
@@ -184,27 +183,21 @@ def test_dynamic_signals_iteration_typing_slicing():
     assert pc[0].edge_index is pc[1].edge_index and pc[1].edge_index is not pc[2].edge_index
 
 
-@pytest.mark.skipif(not refload.available(), reason="/root/reference not present")
-def test_dynamic_signals_match_reference():
+def test_dynamic_signals_match_reference(ref):
     eis, ews, xs, ys, bs, marks = _dynamic_case(seed=3)
     pairs = [
-        (refload.load("signal.dynamic_graph_temporal_signal").DynamicGraphTemporalSignal, DynamicGraphTemporalSignal, (eis, ews, xs, ys)),
-        (refload.load("signal.dynamic_graph_static_signal").DynamicGraphStaticSignal, DynamicGraphStaticSignal, (eis, ews, xs[0], ys)),
-        (refload.load("signal.dynamic_graph_temporal_signal_batch").DynamicGraphTemporalSignalBatch, DynamicGraphTemporalSignalBatch, (eis, ews, xs, ys, bs)),
-        (refload.load("signal.dynamic_graph_static_signal_batch").DynamicGraphStaticSignalBatch, DynamicGraphStaticSignalBatch, (eis, ews, xs[0], ys, bs)),
-        (refload.load("signal.static_graph_temporal_signal_batch").StaticGraphTemporalSignalBatch, StaticGraphTemporalSignalBatch, (eis[0], ews[0], xs, ys, bs[0])),
+        (DynamicGraphTemporalSignal, (eis, ews, xs, ys)),
+        (DynamicGraphStaticSignal, (eis, ews, xs[0], ys)),
+        (DynamicGraphTemporalSignalBatch, (eis, ews, xs, ys, bs)),
+        (DynamicGraphStaticSignalBatch, (eis, ews, xs[0], ys, bs)),
+        (StaticGraphTemporalSignalBatch, (eis[0], ews[0], xs, ys, bs[0])),
     ]
-    for ref_cls, our_cls, args in pairs:
-        want, got = ref_cls(*args, marks=marks), our_cls(*args, marks=marks)
-        assert want.snapshot_count == got.snapshot_count
-        for a, b in zip(want, got):
-            for key in ("x", "edge_index", "edge_attr", "y", "marks"):
-                ta, tb = getattr(a, key), getattr(b, key)
-                assert ta.dtype == tb.dtype and torch.equal(ta, tb)
-            if hasattr(a, "batch") and a.batch is not None:
-                assert torch.equal(a.batch, b.batch)
-        wa, ga = want[1:4], got[1:4]
-        assert wa.snapshot_count == ga.snapshot_count and torch.equal(wa[0].x, ga[0].x) and torch.equal(wa[2].edge_index, ga[2].edge_index)
+    for our_cls, args in pairs:
+        want, got = ref["dynamic_signals"][our_cls.__name__], our_cls(*args, marks=marks)
+        keys = ("x", "edge_index", "edge_attr", "y", "marks") + (("batch",) if "Batch" in our_cls.__name__ else ())
+        assert [[_digest(getattr(b, k)) for k in keys] for b in got] == want["snapshots"]
+        ga = got[1:4]
+        assert [ga.snapshot_count, _digest(ga[0].x), _digest(ga[2].edge_index)] == want["slice"]
 
 
 # ---- host-side algebra of the hand-written DCRNN backward ---------------------------------------------------------------

@@ -1,10 +1,12 @@
 """Data-feed parity (CPU): the signal iterator and index-batching follow the reference's semantics;
 indexing is BIT-EXACT (mirrors test/index_test.py:93-114 and test/dataset_test.py:74-171,717-735)."""
+import os
+
 import numpy as np
 import pytest
 import torch
 
-from oracle import refload, signal as OS
+from oracle import signal as OS
 from pytorch_geometric_temporal_b200.dataset import ChickenpoxDatasetLoader
 from pytorch_geometric_temporal_b200.signal import (IndexDataset, StaticGraphTemporalSignal, index_splits, shard_indices,
                                                     temporal_signal_split)
@@ -76,7 +78,7 @@ def test_index_batching_equals_snapshot_iterator_chickenpox():
     assert dataset.snapshot_count == 517
 
 
-def test_index_dataset_matches_oracle_and_reference():
+def test_index_dataset_matches_oracle_and_reference(golden_dir):
     rng = np.random.RandomState(0)
     data = rng.rand(60, 7, 2).astype(np.float32)
     tr, va, te = index_splits(60, 12)
@@ -87,10 +89,11 @@ def test_index_dataset_matches_oracle_and_reference():
         x, y = ds[i]
         ox, oy = OS.index_window(data, tr, i, 12)
         assert np.array_equal(x.numpy(), ox) and np.array_equal(y.numpy(), oy)
-    if refload.available():
-        ref = refload.load("signal.index_dataset").IndexDataset(tr, data, 12)
-        for i in range(len(ds)):
-            assert torch.equal(ds[i][0], ref[i][0]) and torch.equal(ds[i][1], ref[i][1])
+    # what the unmodified reference IndexDataset returns for every window (tests/golden/make_goldens_parity.py)
+    ref = torch.load(os.path.join(golden_dir, "reference_data.pt"), weights_only=False)["index_dataset"]
+    assert len(ds) == len(ref["x"])
+    for i in range(len(ds)):
+        assert torch.equal(ds[i][0], ref["x"][i]) and torch.equal(ds[i][1], ref["y"][i])
     with pytest.raises(ValueError):
         IndexDataset(tr, data, 12, lazy=True)
 
