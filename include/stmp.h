@@ -293,14 +293,18 @@ int stmp_gru_bwd_zr(int64_t B, int64_t N, int64_t cin, int64_t cout, int64_t du_
  *   stmp_gemm_packed_elems(K,N): number of fp16 elements of the packed weight buffer
  *   stmp_gemm_prepack: W [K,N] row-major (row stride ldw) -> packed (hi/lo, K-major, K padded to 64); once per weight update
  *   stmp_gemm_f32: A row-major (row stride lda), C row-major (ldc); needs N <= 256, N % 32 == 0, K % 4 == 0, 16-byte aligned
- *                  rows; otherwise STMP_EUNSUPPORTED (callers use cuBLAS)
+ *                  rows; otherwise STMP_EUNSUPPORTED (callers use cuBLAS).  The split holds a relative 2^-22 only for operands in
+ *                  2^-3 <= |v| < 65520 (absolute ~2^-25 below, inf above).  a_row_scale (optional, [M] powers of two that fp32
+ *                  holds together with their reciprocals): row r of A is multiplied by a_row_scale[r] before the split and the
+ *                  row of the product by 1/a_row_scale[r] before the bias -- both exact; lets a caller bring every row of an
+ *                  operand of arbitrary magnitude into the split's range.
  *   stmp_gemm_lstm_f32: same contraction with N = 4*cout (column blocks i|f|c|o) fused with the peephole-LSTM gate epilogue
  *                  of GConvLSTM (gconv_lstm.py:168-202): conv_bias [4*cout] (ChebConv biases), cell C_{t-1} [M,cout],
  *                  peepholes w_c{i,f,o} [cout], gate biases b_{i,f,c,o} [cout] -> h_out, c_out [M,cout]; cout in {32, 64}. */
 int64_t stmp_gemm_packed_elems(int64_t K, int64_t N);
 int stmp_gemm_prepack(const float* W, int64_t ldw, int64_t K, int64_t N, void* packed, void* stream);
 int stmp_gemm_f32(const float* A, int64_t lda, int64_t M, int64_t K, int64_t N, const void* packed, const float* bias,
-                  float* C, int64_t ldc, void* stream);
+                  const float* a_row_scale, float* C, int64_t ldc, void* stream);
 int stmp_gemm_lstm_f32(const float* A, int64_t lda, int64_t M, int64_t K, int64_t cout, const void* packed,
                        const float* conv_bias, const float* cell, const float* wci, const float* wcf, const float* wco,
                        const float* bi, const float* bf, const float* bc, const float* bo, float* h_out, float* c_out,

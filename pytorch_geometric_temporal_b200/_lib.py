@@ -76,7 +76,7 @@ _SIGNATURES = {
     "stmp_lstm_oh": (c_int, [c_int64, c_int64, _P, _P, _P, _P, _P, _P, _P]),
     "stmp_gemm_packed_elems": (c_int64, [c_int64, c_int64]),
     "stmp_gemm_prepack": (c_int, [_P, c_int64, c_int64, c_int64, _P, _P]),
-    "stmp_gemm_f32": (c_int, [_P, c_int64, c_int64, c_int64, c_int64, _P, _P, _P, c_int64, _P]),
+    "stmp_gemm_f32": (c_int, [_P, c_int64, c_int64, c_int64, c_int64, _P, _P, _P, _P, c_int64, _P]),
     "stmp_gemm_lstm_f32": (c_int, [_P, c_int64, c_int64, c_int64, c_int64, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "stmp_window_gather": (c_int, [_P, c_int64, c_int64, _P, c_int64, c_int64, _P, _P, _P]),
     "stmp_set_option": (c_int, [c_char_p, c_int]),

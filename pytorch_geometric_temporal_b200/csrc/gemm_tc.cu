@@ -10,6 +10,12 @@
 // write both halves into the hand-swizzled K-major SWIZZLE_128B layout the UMMA descriptors expect.  Two stages:
 // the tile of k-block i+1 is loaded/converted while the MMAs of k-block i run (tcgen05.commit -> mbarrier).
 //
+// The split keeps a relative 2^-22 only while an operand lies in 2^-3 <= |v| < 65520: below 2^-3 `lo` is subnormal and the
+// error of the split is an absolute ~2^-25, below ~3e-8 a value is 0 in both halves, and |v| >= 65520 becomes inf.  Operands of
+// unknown magnitude (gradients) go through `a_row_scale`: row r of A is multiplied by the power of two a_row_scale[r] while it is
+// staged and the row of the product by its reciprocal in the epilogue -- both exact, so the result does not depend on the scale of
+// the row as long as fp32 holds it.
+//
 // One CTA = 128 rows x all N (<= 256) columns, so A is read from HBM exactly once: algorithmic bytes
 // 4*M*K + 4*M*N (+ the L2-resident weights).  This is a true dense GEMM (cfg5: 80 000 x 384 x 256), the one place on
 // the path where tensor cores are the right tool (north_star).
@@ -30,6 +36,7 @@ struct GemmParams {
   const __half* w_hi;   // [N][Kpad]
   const __half* w_lo;
   const float* bias;    // [N] or null
+  const float* a_scale; // [M] powers of two or null (EPI == 0 only): C[r] = ((a_scale[r] * A[r]) @ W) / a_scale[r] + bias
   float* C; long long ldc;
   // LSTM epilogue (EPI == 1): N = 4*Co, column blocks i|f|c|o
   int Co;
@@ -79,6 +86,12 @@ __global__ void __launch_bounds__(GM_NT, 1) k_gemm_split(const GemmParams p) {
   const uint32_t idesc = umma_idesc_f16(128, N);
 
   float4 av[8];
+  float ascale[8];   // the row scale of each of this thread's 8 staging rows (row idx >> 4 = tid / 16 + 16 j)
+#pragma unroll
+  for (int j = 0; j < 8; ++j) {
+    const long long row = m0 + ((tid + j * GM_NT) >> 4);
+    ascale[j] = (EPI == 0 && p.a_scale && row < p.M) ? __ldg(p.a_scale + row) : 1.f;
+  }
   auto load_a = [&](int kb) {
     const int k0 = kb * GM_BK;
 #pragma unroll
@@ -89,6 +102,7 @@ __global__ void __launch_bounds__(GM_NT, 1) k_gemm_split(const GemmParams p) {
       const int k = k0 + 4 * c4;
       av[j] = make_float4(0.f, 0.f, 0.f, 0.f);
       if (row < p.M && k < p.K) av[j] = __ldg(reinterpret_cast<const float4*>(p.A + row * p.lda + k));   // K % 4 == 0
+      if (EPI == 0 && p.a_scale) { av[j].x *= ascale[j]; av[j].y *= ascale[j]; av[j].z *= ascale[j]; av[j].w *= ascale[j]; }
     }
   };
 
@@ -165,6 +179,7 @@ __global__ void __launch_bounds__(GM_NT, 1) k_gemm_split(const GemmParams p) {
   const uint32_t trow = tmem + ((uint32_t)(q * 32) << 16);
   if (EPI == 0) {
     const int ncol = N / 2;   // N % 32 == 0 on this path
+    const float unscale = (p.a_scale && live) ? __frcp_rn(__ldg(p.a_scale + row)) : 1.f;   // exact: a power of two
     for (int c0 = half * ncol; c0 < (half + 1) * ncol; c0 += 16) {
       uint32_t v[16];
       tmem_ld16(trow + c0, v);
@@ -175,6 +190,7 @@ __global__ void __launch_bounds__(GM_NT, 1) k_gemm_split(const GemmParams p) {
         for (int j = 0; j < 4; ++j) {
           float4 o = make_float4(__uint_as_float(v[4 * j]), __uint_as_float(v[4 * j + 1]), __uint_as_float(v[4 * j + 2]),
                                  __uint_as_float(v[4 * j + 3]));
+          if (p.a_scale) { o.x *= unscale; o.y *= unscale; o.z *= unscale; o.w *= unscale; }
           if (p.bias) {
             const float4 bq = __ldg(reinterpret_cast<const float4*>(p.bias + c0 + 4 * j));
             o.x += bq.x; o.y += bq.y; o.z += bq.z; o.w += bq.w;
@@ -268,7 +284,7 @@ extern "C" int stmp_gemm_prepack(const float* W, int64_t ldw, int64_t K, int64_t
 }
 
 extern "C" int stmp_gemm_f32(const float* A, int64_t lda, int64_t M, int64_t K, int64_t N, const void* packed, const float* bias,
-                             float* C, int64_t ldc, void* stream) {
+                             const float* a_row_scale, float* C, int64_t ldc, void* stream) {
   STMP_REQUIRE(A && packed && C, STMP_EINVAL, "stmp_gemm_f32: NULL pointer");
   int rc = gemm_check(M, K, N, A, lda);
   if (rc) return rc;
@@ -277,7 +293,7 @@ extern "C" int stmp_gemm_f32(const float* A, int64_t lda, int64_t M, int64_t K, 
   GemmParams p = {};
   p.A = A; p.lda = lda; p.M = (int)M; p.K = (int)K; p.N = (int)N; p.Kpad = (int)((K + GM_BK - 1) / GM_BK * GM_BK);
   p.w_hi = reinterpret_cast<const __half*>(packed); p.w_lo = p.w_hi + N * p.Kpad;
-  p.bias = bias; p.C = C; p.ldc = ldc;
+  p.bias = bias; p.a_scale = a_row_scale; p.C = C; p.ldc = ldc;
   return gemm_launch<0>(p, (cudaStream_t)stream);
 }
 

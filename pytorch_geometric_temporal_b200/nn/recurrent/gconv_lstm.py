@@ -30,7 +30,7 @@ class _LstmCellFn(torch.autograd.Function):
     forward : Chebyshev basis S = [T_0|..|T_{K-1}]([X|H]) built in place by `stmp_spmm`, then ONE tcgen05 launch computes S @ W and
               the whole peephole gate chain in its epilogue (`stmp_gemm_lstm_f32`).  Only S, C_{t-1}, C_t are kept.
     backward: pre = S @ W recomputed on tcgen05 -> `stmp_lstm_gate_bwd` (gate derivatives) -> dS = dpre @ W^T (tcgen05, two column
-              halves) -> adjoint of the Chebyshev recurrence by TRANSPOSED SpMMs in place -> dX, dH;  dW = S^T dpre as a chunked
+              halves, rows of dpre scaled by powers of two into the split's range) -> adjoint of the Chebyshev recurrence by TRANSPOSED SpMMs in place -> dX, dH;  dW = S^T dpre as a chunked
               GEMM; peephole / bias gradients as column reductions.  ~14 launches instead of the ~90 autograd records."""
 
     @staticmethod
@@ -64,8 +64,11 @@ class _LstmCellFn(torch.autograd.Function):
         dS = torch.empty_like(S)
         dS2 = dS.view(rows, KCw)
         half = KCw // 2
-        for j in range(2):                                                                 # dS = dpre @ W^T, N split in two (N <= 256)
-            ops.gemm(dpre, ctx.packedT[j], 4 * Co, half, None, out=dS2[:, j * half:(j + 1) * half])
+        # dS = dpre @ W^T, N split in two (N <= 256).  dpre is a gradient: its magnitude follows the loss (a mean over 10^6 terms, a
+        # loss scale), so every row is scaled by a power of two into the range of the fp16 hi/lo split and back (exact).
+        rs = ops.pow2_row_scale(dpre)
+        for j in range(2):
+            ops.gemm(dpre, ctx.packedT[j], 4 * Co, half, None, out=dS2[:, j * half:(j + 1) * half], row_scale=rs)
         dW = _chunked_tn(S2, dpre) if ctx.needs_input_grad[3] else None
         colsum = dpre.sum(0)
         dcb = colsum if ctx.has_cb else None

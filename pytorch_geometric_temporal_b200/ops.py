@@ -258,12 +258,31 @@ def gemm_prepack(W: torch.Tensor) -> torch.Tensor:
     return packed
 
 
+def pow2_row_scale(A: torch.Tensor) -> torch.Tensor:
+    """Per-row powers of two s_r = 2^(12 - E_r), E_r the binary exponent of max|A_r|, for `gemm(..., row_scale=)`: they bring each
+    row's largest magnitude into [2^12, 2^13), where the fp16 hi/lo split keeps its relative 2^-22.  The shift is clamped to +-126 so
+    s_r and 1/s_r are normal fp32 (zero and subnormal rows get 2^126; zero rows stay zero), and a row holding inf / NaN gets a finite
+    scale (and stays non-finite).  Read off the exponent bits of the row max: one reduction and four elementwise launches on
+    (M,) values.  A (M, K) fp32 on any device -> (M,) fp32."""
+    amax = torch.linalg.vector_norm(A, float("inf"), dim=-1)
+    biased = amax.view(torch.int32) >> 23                           # E + 127; 0 for zero / subnormal, 255 for inf / NaN
+    return ((266 - biased).clamp_(1, 253) << 23).view(torch.float32)   # the IEEE bits of 2^(12 - E), E + 127 in [1, 253]
+
+
 def gemm(A: torch.Tensor, packed: torch.Tensor, K: int, N: int, bias: Optional[torch.Tensor] = None,
-         out: Optional[torch.Tensor] = None) -> torch.Tensor:
+         out: Optional[torch.Tensor] = None, row_scale: Optional[torch.Tensor] = None) -> torch.Tensor:
     """C = A @ W + bias on tcgen05 with the fp16 hi/lo operand split (fp32-class accuracy).  A (..., K) contiguous.
-    `out`: a 2-D (M, N) view with unit column stride (e.g. a column block of a wider buffer) to write into."""
+    `out`: a 2-D (M, N) view with unit column stride (e.g. a column block of a wider buffer) to write into.
+    The split is exact to a relative 2^-22 only for 2^-3 <= |a| < 65520; below that its error is an absolute ~2^-25 (values under
+    ~3e-8 vanish) and from 65520 up the operand is inf.  For an A of arbitrary magnitude (a gradient) pass
+    `row_scale = pow2_row_scale(A)`: every row is scaled into that range before the split and back after the product, exactly, so
+    the result is the same for any power-of-two scaling of A."""
     A = _f32c(A, "A")
     M = A.numel() // K
+    if row_scale is not None:
+        row_scale = _f32c(row_scale, "row_scale")
+        if row_scale.numel() != M:
+            raise RuntimeError(f"gemm: row_scale must have one entry per row of A ({M}), got {row_scale.numel()}")
     if out is None:
         C = torch.empty(*A.shape[:-1], N, dtype=torch.float32, device=A.device)
         ldc = N
@@ -274,7 +293,8 @@ def gemm(A: torch.Tensor, packed: torch.Tensor, K: int, N: int, bias: Optional[t
         ldc = C.stride(0)
     b = None if bias is None else _f32c(bias.detach(), "bias")
     with torch.cuda.device(A.device):
-        _lib.check(_lib.lib().stmp_gemm_f32(_lib.ptr(A), K, M, K, N, _lib.ptr(packed), _lib.ptr(b), _lib.ptr(C), ldc, _lib.stream_ptr()))
+        _lib.check(_lib.lib().stmp_gemm_f32(_lib.ptr(A), K, M, K, N, _lib.ptr(packed), _lib.ptr(b), _lib.ptr(row_scale), _lib.ptr(C), ldc,
+                                            _lib.stream_ptr()))
     return C
 
 

@@ -1,9 +1,10 @@
 """Host-side algebra of the hand-written GConvLSTM cell backward (`nn/recurrent/gconv_lstm.py::_LstmCellFn`) checked on the CPU
 against autograd through the op-for-op path and against the reference module's gradients: the CUDA entry points are replaced by
 dense torch stand-ins that follow the contracts of include/stmp.h (stmp_spmm on column blocks, stmp_gemm_lstm_f32, stmp_gemm_f32
-with a strided `out`, stmp_lstm_gate_bwd).  Pins, without a GPU: the recompute-in-backward scheme, the gate derivatives' call
-shapes, dS = dpre W^T in two column halves, the in-place adjoint of the Chebyshev recurrence, the chunked weight gradient, the
-peephole / bias reductions and the reuse of one (W, bias) graph across the steps of a sequence."""
+with a strided `out` and `a_row_scale`, stmp_lstm_gate_bwd).  Pins, without a GPU: the recompute-in-backward scheme, the gate
+derivatives' call shapes, dS = dpre W^T in two column halves on power-of-two row-scaled dpre, the in-place adjoint of the Chebyshev
+recurrence, the chunked weight gradient, the peephole / bias reductions and the reuse of one (W, bias) graph across the steps of a
+sequence."""
 import pytest
 import torch
 
@@ -33,8 +34,14 @@ def _install(monkeypatch):
     def gemm_prepack(W):
         return W.clone()                                  # "packed" = the fp32 matrix itself
 
-    def gemm(A, packed, K, N, bias=None, out=None):
-        C = A.reshape(-1, K) @ packed
+    def gemm(A, packed, K, N, bias=None, out=None, row_scale=None):
+        A2 = A.reshape(-1, K)
+        if row_scale is None:
+            C = A2 @ packed
+        else:                                             # a_row_scale: one power of two per row of A, undone on the product
+            assert row_scale.shape == (A2.size(0),) and (torch.frexp(row_scale).mantissa == 0.5).all()
+            row_scaled_calls.append(A2.size(0))
+            C = ((A2 * row_scale[:, None]) @ packed) / row_scale[:, None]
         if bias is not None:
             C = C + bias
         if out is not None:
@@ -60,6 +67,7 @@ def _install(monkeypatch):
         dpi, dpf, dpc = dcn * tv * iv * (1 - iv), dcn * c_old * fv * (1 - fv), dcn * iv * (1 - tv * tv)
         return torch.cat([dpi, dpf, dpc, dpo], dim=1), dcn * fv + dpi * wci + dpf * wcf
 
+    row_scaled_calls = []
     for name, fn in dict(spmm_cols=spmm_cols, spmm=spmm, gemm_prepack=gemm_prepack, gemm=gemm, gemm_lstm=gemm_lstm,
                          lstm_gate_bwd=lstm_gate_bwd).items():
         monkeypatch.setattr(ops, name, fn)
@@ -71,11 +79,12 @@ def _install(monkeypatch):
         M.index_put_((e[1], e[0]), w, accumulate=True)
         return _Plan(M)
     monkeypatch.setattr(cheb_mod.ChebPlanMixin, "_cheb_plan", plan)
+    return row_scaled_calls
 
 
 @pytest.mark.parametrize("K,batched", [(3, False), (2, True), (1, False)])
-def test_lstm_cell_backward_matches_autograd_and_reference(monkeypatch, K, batched):
-    _install(monkeypatch)
+def test_lstm_cell_backward_row_scaled_matches_autograd_and_reference(monkeypatch, K, batched):
+    row_scaled_calls = _install(monkeypatch)
     torch.manual_seed(K)
     n, Ci, Co, T = 24, 32, 32, 3
     ei = torch.stack([torch.randint(0, n, (90,)), torch.randint(0, n, (90,))])
@@ -100,6 +109,7 @@ def test_lstm_cell_backward_matches_autograd_and_reference(monkeypatch, K, batch
         loss.backward()
         outs[name] = (H.detach(), C.detach(), x.grad, {k: p.grad.clone() for k, p in m.named_parameters()})
     assert a._train_cache is None                                   # the shared (W, bias) graph was dropped by the backward pass
+    assert len(row_scaled_calls) == 2 * T                           # every step's dS = dpre W^T (two halves) took row-scaled dpre
     fH, fC, fx, fp = outs["fused"]
     aH, aC, ax, ap = outs["autograd"]
     assert torch.allclose(fH, aH, rtol=1e-5, atol=1e-6) and torch.allclose(fC, aC, rtol=1e-5, atol=1e-6)
